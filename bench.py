@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our CUDA path (one process per GPU under torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K ...  the reference's own CPU implementation on the host cores
+  --dump-outputs DIR                                       also write what the last timed step computed, as DIR/<name>.npy
 
 Workload (BASELINE.json configs[1]): 65,536 random boxes dropped onto a ground plane, 8 solver iterations, measured on the
 settled pile.  One "step" = one sub-step of example/main.cpp:274-328.  Prints ONE JSON line (see README / DESIGN.md §5)."""
@@ -152,6 +153,8 @@ def run_sharded(args, rank, world, local):
     import torch.distributed as dist
     import nudge_b200
     from nudge_b200 import shard
+    if args.dump_outputs:
+        raise SystemExit("--dump-outputs: not available for a scene sharded across GPUs (use --replicas, or one GPU)")
     side = torch.cuda.Stream()                     # a capturable stream: nb_shard_step records the step into a CUDA graph there
     torch.cuda.set_stream(side)
     stream = side.cuda_stream
@@ -374,6 +377,8 @@ def run_ours(args):
     if prof and prof != "staged":
         torch.cuda.profiler.stop()
     launches = sim.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_bodies(sim, args.dump_outputs)
     if world > 1: dist.barrier()
     sampler.stop_flag = True
     step_ms = [a.elapsed_time(b) for a, b in step_ev]
@@ -483,6 +488,18 @@ def run_ours(args):
     if world > 1: dist.destroy_process_group()
 
 
+def dump_bodies(sim, out_dir):
+    """What a caller of nb_step receives after the last timed step (nb_download_bodies): every body's transform, momentum and idle counter,
+    float32, one .npy per field: 3.7 MB for the default 65,537 bodies, 59 MB for the largest config (c4).  The scene and its settling are
+    seeded, so two builds given the same arguments can be compared file for file.  Under --replicas, rank 0's scene."""
+    sim.download_bodies()
+    os.makedirs(out_dir, exist_ok=True)
+    fields = {"position": sim.transforms["position"], "rotation": sim.transforms["rotation"], "velocity": sim.momentum["velocity"],
+              "angular_velocity": sim.momentum["angular_velocity"], "idle_counter": sim.idle}
+    for name, a in fields.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def throughput_leg(sim, scene, flush, K):
     """The workload of the line, continued from the state the timed loop left, with nb_set_solver_mode(NB_SOLVER_THROUGHPUT): same
     timing rules (L2 flush between steps, CUDA events around nb_step), and the roofline of ITS dominant kernel, k_jacobi_sweep, from
@@ -549,6 +566,8 @@ def cpu_baseline_sample(args):
     8191-box pile of the same generator (the reference's 2^13 collider limit, nudge.cpp:3010), settled on the GPU, then timed."""
     import nudge_b200
     from oracle import pyref
+    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libnudge_ref_fast.so")):
+        return None                               # the reference is not built in this tree (oracle/Makefile needs its sources)
     s = CONFIGS[args.config]["small"](args, 77)
     g = nudge_b200.Sim(s)
     settle_gpu(g, args.presim)
@@ -605,7 +624,7 @@ def run_reference(args):
     work(make)
     for _ in range(max(args.warmup, 1)):
         work(step)
-    K = min(args.steps, args.ref_steps)
+    K = args.steps
     t0 = time.perf_counter()
     for _ in range(K):
         work(step)
@@ -637,7 +656,6 @@ def main():
     ap.add_argument("--iterations", type=int, default=0, help="solver sweeps per step (0 = the config's own)")
     ap.add_argument("--presim", type=int, default=-1, help="untimed settling steps before the measurement (-1 = the config's own)")
     ap.add_argument("--ref-presim", type=int, default=700)
-    ap.add_argument("--ref-steps", type=int, default=40)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-throughput-leg", action="store_true", help="skip the extra throughput-mode measurement of the same scene (key throughput_mode)")
     ap.add_argument("--solver", default="parity", choices=["parity", "throughput"], help="parity = the reference's exact Gauss-Seidel order (default, bit-identical results); throughput = mass-splitting Jacobi")
@@ -645,7 +663,12 @@ def main():
     ap.add_argument("--margin", type=float, default=0.5, help="N > 1: extra halo width beyond the bounding radii (room for motion between re-partitions)")
     ap.add_argument("--no-parity-check", action="store_true", help="N > 1: skip the NCCL / peer / host-exchange bit-equality check before the timed region")
     ap.add_argument("--replicas", action="store_true", help="N > 1: run N independent copies of the workload instead of one sharded scene")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the bodies' state after the last timed step as DIR/<field>.npy (float32; one scene per GPU only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; the reference arm has none")
     if args.presim < 0:
         args.presim = CONFIGS[args.config]["presim"]
     if args.impl == "reference":

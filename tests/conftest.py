@@ -15,10 +15,3 @@ def _build_oracle():
     """The CPU restatement is test infrastructure: build it if the prebuilt file did not travel."""
     if not os.path.exists(os.path.join(ROOT, "oracle", "liboracle.so")):
         subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "oracle"])
-
-
-def have_ref():
-    return os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libnudge_ref.so"))
-
-
-needs_ref = pytest.mark.skipif(not have_ref(), reason="oracle/_ref not built (needs /root/reference in the build container)")

@@ -33,16 +33,25 @@ def random_scene(rng):
     return s
 
 
+def contact_capacity(s):
+    return 256 * s.n_bodies + 4096
+
+
+def maybe_sleep(rng, sims):
+    """Before a step: now and then put a random half of the scene to sleep in every sim of `sims`."""
+    if rng.random() < 0.05:
+        m = rng.random(sims[0].scene.n_bodies) < 0.5
+        for x in sims:
+            x.idle[m] = 0xff
+            x.momentum["velocity"][m] = 0; x.momentum["angular_velocity"][m] = 0
+
+
 def run_scene(s, rng, steps):
     """Returns None, or a description of the first difference."""
     from oracle import pyref, pyoracle
-    r = pyref.RefSim(s, contact_capacity=256 * s.n_bodies + 4096, arena_mb=1024); o = pyoracle.OracleSim(s, contact_capacity=r.cap)
+    r = pyref.RefSim(s, contact_capacity=contact_capacity(s), arena_mb=1024); o = pyoracle.OracleSim(s, contact_capacity=r.cap)
     for i in range(steps):
-        if rng.random() < 0.05:      # put part of the scene to sleep
-            m = rng.random(s.n_bodies) < 0.5
-            r.idle[m] = 0xff; o.idle[m] = 0xff
-            for x in (r, o):
-                x.momentum["velocity"][m] = 0; x.momentum["angular_velocity"][m] = 0
+        maybe_sleep(rng, (r, o))
         rep = Report("%s step %d" % (s.name, i))
         if not compare_ref_oracle_step(r, o, rep):
             return str(rep)

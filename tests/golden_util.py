@@ -64,3 +64,40 @@ def demo_scene(g, state="initial"):
 def demo_substeps(frame):
     """simulate() calls behind recorded frame f: f + 1, two sub-steps each (example/main.cpp:275, 330-334)."""
     return 2 * (frame + 1)
+
+
+# ---- every stage of every step of the reference, as digests (tests/golden/make_ref_traces.py, parity_util.ref_layout_stages) ----
+def load_ref_traces():
+    return np.load(os.path.join(HERE, "golden", "ref_traces.npz"))
+
+
+def _sleep_after(step, seed, share):
+    """Hook: before `step`, put a seeded random `share` of the bodies to sleep (idle counter 0xff, momentum zeroed)."""
+    def hook(i, sim):
+        if i == step:
+            m = np.random.default_rng(seed).random(sim.scene.n_bodies) < share
+            sim.idle[m] = 0xff
+            sim.momentum["velocity"][m] = 0; sim.momentum["angular_velocity"][m] = 0
+    return hook
+
+
+def ref_trace_cases(name):
+    """Yields (case, scene, steps, contact capacity, hook(i, sim) run before step i) for the traces of test_oracle_vs_ref.py's `name`.
+    The fuzz cases share one generator and must be run in order, each to the end, before the next is drawn."""
+    cap = lambda s: max(1024, 64 * s.n_bodies)
+    if name == "small_mixed":
+        s = S.demo_scene(100, 100, iterations=4, spread=2.0, height=20.0); yield name, s, 30, cap(s), None
+    elif name == "demo_config0":
+        s = S.demo_scene(1024, 1024, iterations=8); yield name, s, 4, cap(s), None
+    elif name == "rotated_box_drop":
+        s = S.box_drop(1500, iterations=8); yield name, s, 12, cap(s), None
+    elif name == "sleeping_islands":
+        s = S.demo_scene(120, 120, iterations=4, spread=6.0, height=6.0, seed=11); yield name, s, 46, cap(s), _sleep_after(40, 5, 0.8)
+    elif name == "fuzz":
+        from tests import fuzz_oracle_vs_ref as F
+        rng = np.random.default_rng(77)
+        for k in range(120):
+            s = F.random_scene(rng)
+            yield "fuzz%03d" % k, s, int(rng.integers(5, 40)), F.contact_capacity(s), (lambda i, sim: F.maybe_sleep(rng, (sim,)))
+    else:
+        raise KeyError(name)

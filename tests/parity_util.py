@@ -1,4 +1,5 @@
 """Stage-by-stage bit comparison helpers shared by the CPU (oracle vs reference) and GPU (CUDA vs oracle) parity tests."""
+import hashlib
 import numpy as np
 from nudge_b200 import abi
 
@@ -47,46 +48,70 @@ def rows_by_contact(view, n_contacts):
                 a=view["a"][first], b=view["b"][first])
 
 
+def ref_layout_stages(x, widened):
+    """Runs one full step of x (the reference's RefSim, or the widened OracleSim with widened=True) and yields (stage, array) after every
+    stage, each array in the reference's uint16 / packed-tag layout, so that the two implementations, or one of them and digests of the
+    other recorded earlier (tests/golden/make_ref_traces.py), compare byte for byte."""
+    tag = (lambda v, t, f: abi.wide_tag_to_ref(v[t], v[f])) if widened else (lambda v, t, f: v[t])
+    u32 = lambda a: np.asarray(a).astype(np.uint32)
+    x.collide()
+    c = x.contacts_view()
+    yield "contact count", np.array([c["count"]], np.uint32)
+    yield "active", u32(c["active"])
+    yield "contacts", c["data"]
+    yield "bodies.a", u32(c["bodies"]["a"])
+    yield "bodies.b", u32(c["bodies"]["b"])
+    yield "tags", tag(c, "tags", "features")
+    yield "sleeping", abi.wide_pair_to_ref(c["sleeping"]) if widened else c["sleeping"]
+    x.apply_gravity_damping()
+    yield "momentum after gravity", x.momentum
+    x.read_cached_impulses()
+    i = x.impulses_view()
+    yield "sorted", i["sorted"]
+    yield "impulses", i["data"]
+    yield "culled tags", tag(i, "culled_tags", "culled_features")
+    yield "culled data", i["culled_data"]
+    x.setup_contact_constraints()
+    k = x.constraints_view()
+    yield "batches", np.array([k["batches"]], np.uint32)
+    yield "constraint_to_contact", k["contact"]
+    yield "rows", k["rows"]
+    yield "warm-start states", k["states"]
+    yield "momentum after setup", x.momentum
+    for it in range(int(x.scene.iterations)):
+        x.apply_impulses()
+        yield "momentum sweep %d" % it, x.momentum
+    yield "states", x.constraints_view()["states"]
+    x.update_cached_impulses()
+    yield "updated impulses", x.impulses_view()["data"]
+    x.write_cached_impulses()
+    cv = x.cache_view()
+    yield "cache tags", tag(cv, "tags", "features")
+    yield "cache data", cv["data"]
+    x.advance()
+    yield "transforms", x.transforms
+    yield "idle", x.idle
+
+
+# stages after which a difference makes the rest of the step meaningless to compare (array lengths follow from them)
+_STOP_AFTER = ("contact count", "sleeping", "batches")
+
+
 def compare_ref_oracle_step(r, o, rep):
     """One full step, the unmodified reference (uint16 layout) against the widened restatement."""
-    r.collide(); o.collide()
-    rc, oc = r.contacts_view(), o.contacts_view()
-    rep.check("contact count", rc["count"] == oc["count"], "%d vs %d" % (rc["count"], oc["count"]))
-    rep.eq("active", rc["active"].astype(np.uint32), oc["active"])
-    if rc["count"] != oc["count"]:
-        return False
-    rep.eq("contacts", rc["data"], oc["data"])
-    rep.eq("bodies.a", rc["bodies"]["a"].astype(np.uint32), oc["bodies"]["a"])
-    rep.eq("bodies.b", rc["bodies"]["b"].astype(np.uint32), oc["bodies"]["b"])
-    rep.eq("tags", rc["tags"], abi.wide_tag_to_ref(oc["tags"], oc["features"]))
-    rep.eq("sleeping", rc["sleeping"], abi.wide_pair_to_ref(oc["sleeping"]))
-    if not rep.ok:
-        return False
-    r.apply_gravity_damping(); o.apply_gravity_damping()
-    rep.eq("momentum after gravity", r.momentum, o.momentum)
-    r.read_cached_impulses(); o.read_cached_impulses()
-    ri, oi = r.impulses_view(), o.impulses_view()
-    rep.eq("sorted", ri["sorted"], oi["sorted"]); rep.eq("impulses", ri["data"], oi["data"])
-    rep.eq("culled tags", ri["culled_tags"], abi.wide_tag_to_ref(oi["culled_tags"], oi["culled_features"]))
-    rep.eq("culled data", ri["culled_data"], oi["culled_data"])
-    r.setup_contact_constraints(); o.setup_contact_constraints()
-    rk, okk = r.constraints_view(), o.constraints_view()
-    if not rep.check("batches", rk["batches"] == okk["batches"], "%d vs %d" % (rk["batches"], okk["batches"])):
-        return False
-    rep.eq("constraint_to_contact", rk["contact"], okk["contact"]); rep.eq("rows", rk["rows"], okk["rows"]); rep.eq("warm-start states", rk["states"], okk["states"])
-    rep.eq("momentum after setup", r.momentum, o.momentum)
-    for it in range(int(r.scene.iterations)):
-        r.apply_impulses(); o.apply_impulses()
-        rep.eq("momentum sweep %d" % it, r.momentum, o.momentum)
-    rep.eq("states", r.constraints_view()["states"], o.constraints_view()["states"])
-    r.update_cached_impulses(); o.update_cached_impulses()
-    rep.eq("updated impulses", r.impulses_view()["data"], o.impulses_view()["data"])
-    r.write_cached_impulses(); o.write_cached_impulses()
-    rcv, ocv = r.cache_view(), o.cache_view()
-    rep.eq("cache tags", rcv["tags"], abi.wide_tag_to_ref(ocv["tags"], ocv["features"])); rep.eq("cache data", rcv["data"], ocv["data"])
-    r.advance(); o.advance()
-    rep.eq("transforms", r.transforms, o.transforms); rep.eq("idle", r.idle, o.idle)
+    for (name, a), (_, b) in zip(ref_layout_stages(r, False), ref_layout_stages(o, True)):
+        rep.eq(name, a, b)
+        if name in _STOP_AFTER and not rep.ok:
+            return False
     return rep.ok
+
+
+def stage_digest(a):
+    """8-byte digest of an array's shape and bytes: what the golden reference traces store per stage."""
+    h = hashlib.blake2b(digest_size=8)
+    h.update(repr(np.shape(a)).encode())
+    h.update(bits(a).tobytes())
+    return np.frombuffer(h.digest(), np.uint64)[0]
 
 
 def compare_oracle_gpu_step(o, g, rep, sweeps_individually=True):

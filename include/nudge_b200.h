@@ -17,6 +17,7 @@
  *   nb_instance_matrices            <- the draw loops of render()          example/main.cpp:224-268 (helpers :53-110)
  *   nb_save_state / nb_load_state   <- the caller-owned PODs               nudge.h:73-129
  *   nb_shard_*                      <- no reference counterpart (the reference is single threaded): SURVEY.md section 8e
+ *   nb_build_query_tree, nb_raycast <- no reference counterpart (ray queries): DESIGN.md section 8.5
  *
  * Data layout: the reference's caller-owned SoA structs (nudge.h:29-129) with every index-carrying field
  * widened to 32 bits (the reference caps at 8192 colliders / 65535 bodies, nudge.cpp:3010, nudge.h:68-71):
@@ -194,6 +195,36 @@ int nb_state_info(const char* path, uint32_t counts[5] /* bodies, boxes, spheres
  * out_is_device != 0: `out` is a device pointer (a mapped GL / Vulkan buffer), the call is asynchronous on `stream`; otherwise `out`
  * is host memory and the call returns when it is filled.  *count = colliders; NB_ERR_CAPACITY if capacity (in matrices) is smaller. */
 int nb_instance_matrices(nb_context*, float* out, uint32_t capacity, int out_is_device, uint32_t* count, void* stream);
+
+/* Ray casts against the device-resident scene (no reference counterpart; nudge_b200/csrc/nb_query_api.cuh, DESIGN.md section 8.5).
+ *
+ * nb_build_query_tree takes a SNAPSHOT of the scene as it is now (body transforms, collider transforms, sizes and tags) into buffers of
+ * its own, allocated on the first call, and builds an 8-ary AABB tree over it; it never touches what the step uses.  nb_raycast queries
+ * the last snapshot, so one build serves any number of ray batches, and rays do not see later nb_advance / nb_step calls until the next
+ * build.  io_is_device != 0: rays and hits are device pointers, the call is asynchronous on `stream` and can be captured into the
+ * caller's own CUDA graph; otherwise they are host pointers, staged through the library's buffers, and the call synchronises.
+ * nb_raycast returns NB_ERR_ARGUMENT when no snapshot exists, when the collider counts changed since it was taken (nb_upload_colliders,
+ * nb_load_state), or when a pointer is null while n > 0.
+ *
+ * Semantics (float32, exact: the same scene and rays give the same bits whatever the tree shape, ray order or launch configuration):
+ *  - The hit is the smallest t in [0, max_t] at which origin + t*direction meets a solid collider.  direction need not be unit length;
+ *    t is measured in units of it.  origin and direction must be finite.
+ *  - Equal t goes to the smallest collider index: boxes 0..nboxes-1, then spheres from nboxes on (the order of nb_instance_matrices).
+ *  - Colliders of body ignore_body are skipped; NB_NO_BODY skips nothing.  Body 0 (the static world) is hit like any other body.
+ *  - An origin inside a collider (boundary included) gives t = 0 and normal = (0,0,0).
+ *  - A miss gives t = max_t, collider = body = tag = NB_NO_BODY and normal = (0,0,0).
+ *  - Collider world transform = body * collider, the operations of the collision stage.
+ *  - Box: the ray is moved into the box frame (origin - position and direction rotated by the conjugate rotation), then slabs against
+ *    the half extents with IEEE division.  A zero direction component makes that axis "inside iff |origin| <= size".  The normal is the
+ *    local axis of the entering slab, signed against the direction and rotated to world space; tied slabs go to the lowest axis (x, y, z).
+ *  - Sphere: m = origin - centre, a = d.d, b = m.d, c = m.m - r*r, disc = b*b - a*c; inside iff c <= 0; otherwise a hit needs disc >= 0,
+ *    a > 0 and t = (-b - sqrt(disc)) / a >= 0, with normal = (origin + t*d - centre) / r.
+ *  The exact order of every float operation is fixed in DESIGN.md section 8.5. */
+typedef struct { float origin[3]; float max_t; float direction[3]; uint32_t ignore_body; } nb_ray;                        /* 32 B */
+typedef struct { float t; uint32_t collider, body, tag; float normal[3]; float unused; } nb_ray_hit;                    /* 32 B */
+#define NB_NO_BODY 0xffffffffu   /* ignore_body: skip nothing.  Also collider / body / tag of a miss */
+int nb_build_query_tree(nb_context*, void* stream);
+int nb_raycast(nb_context*, const nb_ray* rays, nb_ray_hit* hits, uint32_t n, int io_is_device, void* stream);
 
 /* Solver mode.  NB_SOLVER_PARITY (default): the reference's exact Gauss-Seidel order (nudge.cpp:4206-4340 schedule, 4640-4855 sweeps),
  * bit-identical impulses.  NB_SOLVER_THROUGHPUT: mass-splitting Jacobi over the same constraint rows (nudge_b200/csrc/nb_jacobi.cuh) -

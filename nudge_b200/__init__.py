@@ -21,7 +21,8 @@ EXPORTS = ["nb_create", "nb_destroy", "nb_last_error", "nb_upload_bodies", "nb_u
            "nb_shard_step", "nb_shard_graph_active", "nb_shard_partition", "nb_shard_debug_no_exchange",
            "nb_set_solver_mode", "nb_get_solver_mode", "nb_debug_timing_enable", "nb_debug_timing",
            "nb_stream_create", "nb_stream_destroy", "nb_stream_synchronize", "nb_save_state", "nb_load_state", "nb_state_info",
-           "nb_upload_constraint_rows", "nb_download_constraint_rows", "nb_instance_matrices", "nb_shard_build_plan", "nb_shard_local_scene"]
+           "nb_upload_constraint_rows", "nb_download_constraint_rows", "nb_instance_matrices", "nb_shard_build_plan", "nb_shard_local_scene",
+           "nb_build_query_tree", "nb_raycast"]
 
 
 class Config(C.Structure):
@@ -92,6 +93,8 @@ def load_library():
         lib.nb_upload_constraint_rows.argtypes = [V, V, C.c_uint32, V]
         lib.nb_download_constraint_rows.argtypes = [V, V, C.c_uint32, V]
         lib.nb_instance_matrices.argtypes = [V, V, C.c_uint32, C.c_int, V, V]
+        lib.nb_build_query_tree.argtypes = [V, V]
+        lib.nb_raycast.argtypes = [V, V, V, C.c_uint32, C.c_int, V]
         lib.nb_shard_build_plan.argtypes = [V, C.c_uint32, V, V, C.c_uint32, C.c_uint32, V, V, V, V, V, V, V, V]
         lib.nb_shard_local_scene.argtypes = [V, C.c_uint32, V, C.c_uint32, C.c_uint32, V, C.c_uint32, V, C.c_uint32, V, V, V, V, V]
         _lib = lib
@@ -106,6 +109,8 @@ class NudgeError(RuntimeError):
 ROW = np.dtype([("a", "<u4"), ("b", "<u4"), ("lin_a", "<f4", 3), ("ang_a", "<f4", 3), ("lin_b", "<f4", 3), ("ang_b", "<f4", 3),
                 ("bias", "<f4"), ("lo", "<f4"), ("hi", "<f4"), ("impulse", "<f4"), ("softness", "<f4"), ("reserved", "<f4")])
 assert ROW.itemsize == 80
+# nb_ray / nb_ray_hit (32 bytes each) and the "no body" marker: defined with the other record types in scenes.py
+RAY, RAY_HIT, NO_BODY, make_rays = scenes.RAY, scenes.RAY_HIT, scenes.NO_BODY, scenes.make_rays
 
 
 def nccl_unique_id():
@@ -360,6 +365,23 @@ class Sim(abi.HostState):
             out = np.zeros((k, 16), np.float32)
         self._ck(self.lib.nb_instance_matrices(self.ctx, abi.ptr(out), len(out), 0, C.byref(n), self.stream), "nb_instance_matrices")
         return out[:n.value]
+
+    # ---- ray casts against a snapshot of the scene (nb_build_query_tree / nb_raycast, include/nudge_b200.h) ----
+    def build_query_tree(self):
+        """Snapshots the scene as it is now (transforms, colliders, sizes, tags) and builds the query tree; asynchronous on the Sim's stream."""
+        self._ck(self.lib.nb_build_query_tree(self.ctx, self.stream), "nb_build_query_tree")
+
+    def raycast(self, origins=None, directions=None, max_t=np.inf, ignore_body=None, rays=None, device_ptr=None, hits_ptr=None, n=0):
+        """Casts rays against the last snapshot.  Host form: origins / directions [n, 3] (or a RAY array as `rays`), max_t and ignore_body
+        scalars or [n] arrays; returns a RAY_HIT array.  Device form: device_ptr = device address of n RAY records, hits_ptr = device
+        address for n RAY_HIT records (e.g. torch tensors' data_ptr()); asynchronous on the Sim's stream, returns None."""
+        if device_ptr is not None:
+            self._ck(self.lib.nb_raycast(self.ctx, C.c_void_p(device_ptr), C.c_void_p(hits_ptr), int(n), 1, self.stream), "nb_raycast")
+            return None
+        r = np.ascontiguousarray(rays if rays is not None else scenes.make_rays(origins, directions, max_t, ignore_body), scenes.RAY)
+        hits = np.zeros(len(r), scenes.RAY_HIT)
+        self._ck(self.lib.nb_raycast(self.ctx, abi.ptr(r) if len(r) else None, abi.ptr(hits) if len(r) else None, len(r), 0, self.stream), "nb_raycast")
+        return hits
 
     # ---- state files (nb_save_state / nb_load_state; tools/nb_replay steps them headless) ----
     def save_state(self, path):

@@ -53,6 +53,13 @@ struct nb_context {
 	cudaStream_t copy_stream; cudaEvent_t ev_up_begin, ev_up_done; bool upload_pending, capture_joined; int copy_overlap;
 	int solve_wide;   // k_solve hands a body's row over with one 256-bit access instead of two 128-bit ones (default; NB_SOLVE_WIDE=0: the 128-bit protocol)
 	nb_constraint_row* urows; u32 urow_cap, urow_n, urow_levels; unsigned long long urow_version; std::vector<u32> urow_level_off, urow_order;
+	// ray-cast snapshot (nb_build_query_tree, nb_query_api.cuh): every buffer its own, allocated on first use, never one the step reads
+	struct Query {
+		bool built; u32 nboxes, nspheres, K;   // collider counts when the snapshot was taken (K = 0: empty scene)
+		nb_transform* world_xf; float4* aabb_min; float4* aabb_max; u32* col_tag; u32* col_body; u32* counts; u64* keybits;
+		u32* order; u32* rank; u64* mkeys; float4* tree_min; float4* tree_max; float4* leaf; SortBuffers sb; Tree T;
+		nb_ray* rays; nb_ray_hit* hits; u32 io_cap;   // staging of host rays / hits
+	} q;
 
 	// scene
 	nb_transform* xf; nb_body_properties* props; nb_body_momentum* mom; uint8_t* idle;
@@ -898,6 +905,7 @@ int nb_debug_read(nb_context* ctx, const char* name, void* dst, size_t max_bytes
 		{ "inertia", ctx->inertia, sizeof(float4) * 2 * ctx->B },
 		{ "row_planes_all", ctx->rows.plane, sizeof(float) * (size_t)ROW_PLANES_TOTAL * ctx->cstride },
 		{ "body_contacts", ctx->jcnt, sizeof(u32) * ctx->B },
+		{ "query_world_xf", ctx->q.world_xf, sizeof(nb_transform) * ctx->q.K },
 	};
 	if (!strcmp(name, "row_stride")) { if (max_bytes < 4) return NB_ERR_ARGUMENT; *(u32*)dst = ctx->cstride; if (bytes) *bytes = 4; return NB_OK; }
 	if (!strcmp(name, "graph_coop")) { if (max_bytes < 4) return NB_ERR_ARGUMENT; *(u32*)dst = ctx->graph_exec ? (ctx->graph_is_coop ? 2u : 1u) : 0u; if (bytes) *bytes = 4; return NB_OK; }
@@ -960,3 +968,4 @@ int nb_debug_rcp(nb_context* ctx, const float* x, float* y, uint32_t n, int rsq)
 #include "nb_state_api.cuh"
 #include "nb_rows_api.cuh"
 #include "nb_render_api.cuh"
+#include "nb_query_api.cuh"

@@ -20,8 +20,24 @@ CONTACT = np.dtype([("position", "<f4", 3), ("penetration", "<f4"), ("normal", "
 IMPULSE = np.dtype([("impulse", "<f4", 3), ("unused", "<f4")])
 PAIR16 = np.dtype([("a", "<u2"), ("b", "<u2")])
 PAIR32 = np.dtype([("a", "<u4"), ("b", "<u4")])
+# nb_ray / nb_ray_hit (include/nudge_b200.h): ray casts against the device-resident scene
+RAY = np.dtype([("origin", "<f4", 3), ("max_t", "<f4"), ("direction", "<f4", 3), ("ignore_body", "<u4")])
+RAY_HIT = np.dtype([("t", "<f4"), ("collider", "<u4"), ("body", "<u4"), ("tag", "<u4"), ("normal", "<f4", 3), ("unused", "<f4")])
+NO_BODY = 0xFFFFFFFF
 
 assert TRANSFORM.itemsize == 32 and MOMENTUM.itemsize == 32 and CONTACT.itemsize == 32
+assert RAY.itemsize == 32 and RAY_HIT.itemsize == 32
+
+
+def make_rays(origins, directions, max_t=np.inf, ignore_body=None):
+    """A RAY array from [n, 3] origins and directions; max_t and ignore_body are scalars or [n] arrays (None: ignore no body)."""
+    o = np.asarray(origins, np.float32).reshape(-1, 3)
+    r = np.zeros(len(o), RAY)
+    r["origin"] = o
+    r["direction"] = np.asarray(directions, np.float32).reshape(-1, 3)
+    r["max_t"] = max_t
+    r["ignore_body"] = NO_BODY if ignore_body is None else ignore_body
+    return r
 
 
 class Scene:
